@@ -11,6 +11,7 @@ there (profiles/r02_exchange_n8_diag.txt); `exchange.exchange_used` says which r
 
 Arms
     python bench.py [--gpus N --steps K --warmup W]          this repo (one process per GPU under torchrun)
+                    [--dump-outputs DIR]                     + the last timed fit's coefficients and intercept as .npy
     python bench.py --impl reference [...]                   the reference's own CPU path: scikit-learn
                                                              LinearRegression.fit (stage_1_train_model.py:105-106)
                                                              on a bounded sample, all host threads, rank 0 only
@@ -293,6 +294,13 @@ def exact_check(ctx, b2, X, y, d, sol, dist, tag: str) -> dict:
     return out
 
 
+def dump_outputs(out_dir: str, coef, b0: float) -> None:
+    """What the timed fit hands its caller: the coefficients and the intercept of the last step."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "coef.npy"), np.asarray(coef, dtype=np.float64))
+    np.save(os.path.join(out_dir, "intercept.npy"), np.array([b0], dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------
 def main() -> None:
     ap = argparse.ArgumentParser()
@@ -309,7 +317,12 @@ def main() -> None:
     ap.add_argument("--no-variants", action="store_true", help="alias of --no-extras")
     ap.add_argument("--precision", default="split", choices=["split", "bf16"],
                     help="tensor-core operand precision: bf16 hi+lo split (default) or a single bf16 operand")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed fit's result to DIR/coef.npy and DIR/intercept.npy (float64); the "
+                         "inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     extras = not (args.no_extras or args.no_variants)
 
@@ -417,6 +430,8 @@ def main() -> None:
     t_host = time.perf_counter() - t_host0
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:      # every rank solves the same all-reduced statistic
+        dump_outputs(args.dump_outputs, coef, b0)
     kernel_ms, kernel_launches = ctx.last_kernel_ms()
     launches = ctx.launch_count() - launches0
     fused_fits = ctx.stats()["fused_fits"] - fused0

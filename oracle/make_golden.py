@@ -1,23 +1,25 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference.  TEST INFRASTRUCTURE ONLY.
 
-Run in the build container (the only place /root/reference exists):
+Run with a checkout of the reference project at hand:
 
-    python oracle/make_golden.py
+    python oracle/make_golden.py REFERENCE_DIR [OUT_DIR]      (OUT_DIR defaults to tests/golden)
 
 What it does
 ------------
-* imports ``/root/reference/mlops_simulation/stage_1_train_model.py`` with ``boto3`` /
+* imports ``REFERENCE_DIR/mlops_simulation/stage_1_train_model.py`` with ``boto3`` /
   ``botocore.exceptions`` stubbed (they are absent from the image and only used for S3 I/O),
 * calls the reference's own ``train_model(data)`` (stage_1_train_model.py:93-108) and
   ``model_metrics`` (:79-90) on seeded datasets drawn with the reference's data-generating
   process (stage_3_synthetic_data_generation.py:36-43),
 * for D > 1 (the reference itself is D = 1) calls the same scikit-learn entry points the
   reference calls (train_test_split / LinearRegression / the three metrics),
-* stores inputs and outputs as small ``.npz`` fixtures.  The GPU box has no /root/reference;
-  tests there read only the fixtures.
+* stores inputs and outputs as small ``.npz`` fixtures; the tests read only the fixtures.  Rows too large to store
+  (over ``MAX_STORED_BYTES``) are kept as the seed and shape they are drawn with plus their SHA-256;
+  ``tests/conftest.py`` draws them again and checks the digest.
 """
 from __future__ import annotations
 
+import hashlib
 import importlib.util
 import os
 import sys
@@ -28,14 +30,14 @@ import pandas as pd
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-GOLD = os.path.join(ROOT, "tests", "golden")
-REF = "/root/reference/mlops_simulation/stage_1_train_model.py"
+REF_MODULE = os.path.join("mlops_simulation", "stage_1_train_model.py")
+MAX_STORED_BYTES = 1_000_000
 
 sys.path.insert(0, ROOT)
 from oracle import ols_oracle as orc  # noqa: E402
 
 
-def load_reference():
+def load_reference(ref_dir: str):
     boto3 = types.ModuleType("boto3")
     botocore = types.ModuleType("botocore")
     exc = types.ModuleType("botocore.exceptions")
@@ -44,15 +46,16 @@ def load_reference():
     sys.modules.setdefault("boto3", boto3)
     sys.modules.setdefault("botocore", botocore)
     sys.modules.setdefault("botocore.exceptions", exc)
-    spec = importlib.util.spec_from_file_location("ref_stage_1", REF)
+    spec = importlib.util.spec_from_file_location("ref_stage_1", os.path.join(ref_dir, REF_MODULE))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
 
 
-def main() -> None:
+def main(ref_dir: str, out_dir: str) -> None:
+    GOLD = out_dir
     os.makedirs(GOLD, exist_ok=True)
-    ref = load_reference()
+    ref = load_reference(ref_dir)
     import sklearn
 
     # ---- D = 1 through the reference's own train_model -------------------------------
@@ -68,7 +71,7 @@ def main() -> None:
                  r_squared=np.float64(metrics["r_squared"].iloc[0]),
                  max_residual=np.float64(metrics["max_residual"].iloc[0]),
                  columns=np.array(list(metrics.columns)),
-                 sklearn_version=np.array(sklearn.__version__), source=np.array(REF + "::train_model"))
+                 sklearn_version=np.array(sklearn.__version__), source=np.array(REF_MODULE + "::train_model"))
         print(tag, model.coef_, model.intercept_, metrics.to_dict("records")[0])
 
     # ---- model_metrics alone -------------------------------------------------------------
@@ -87,7 +90,10 @@ def main() -> None:
                                    ("n3k_d128_f32", 3_000, 128, 23, np.float32)):
         X, y = orc.generate_dataset(n, d, seed=seed, dtype=dtype)
         out = orc.train_model_sklearn(X, y)
-        np.savez(os.path.join(GOLD, f"sk_train_model_{tag}.npz"), X=X, y=y,
+        rows = {"X": X} if X.nbytes <= MAX_STORED_BYTES else {
+            "seed": np.int64(seed), "X_shape": np.array(X.shape, dtype=np.int64),
+            "X_sha256": np.array(hashlib.sha256(X.tobytes()).hexdigest())}
+        np.savez(os.path.join(GOLD, f"sk_train_model_{tag}.npz"), **rows, y=y,
                  coef=out["coef"], intercept=np.float64(out["intercept"]), rank=np.int64(out["rank"]),
                  singular=out["singular"], MAPE=np.float64(out["MAPE"]),
                  r_squared=np.float64(out["r_squared"]), max_residual=np.float64(out["max_residual"]),
@@ -119,4 +125,6 @@ def main() -> None:
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) not in (2, 3):
+        raise SystemExit("usage: python oracle/make_golden.py REFERENCE_DIR [OUT_DIR]")
+    main(sys.argv[1], sys.argv[2] if len(sys.argv) == 3 else os.path.join(ROOT, "tests", "golden"))

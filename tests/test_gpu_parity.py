@@ -518,9 +518,9 @@ def test_train_model_matches_reference_golden(golden_dir, tag):
 
 
 @pytest.mark.parametrize("tag", ["n10k_d8", "n4k_d32_f32", "n3k_d128_f32"])
-def test_train_model_multi_feature_golden(golden_dir, tag):
+def test_train_model_multi_feature_golden(golden, tag):
     import pandas as pd
-    g = np.load(os.path.join(golden_dir, f"sk_train_model_{tag}.npz"))
+    g = golden(f"sk_train_model_{tag}.npz")
     d = g["X"].shape[1]
     df = pd.DataFrame(g["X"], columns=[f"X{j}" for j in range(d)])
     df["y"] = g["y"]

@@ -35,9 +35,9 @@ def test_metrics_match_reference_golden(golden_dir):
 
 
 @pytest.mark.parametrize("tag,tol", [("n10k_d8", 1e-11), ("n4k_d32_f32", 2e-5), ("n3k_d128_f32", 2e-4)])
-def test_train_model_multi_feature_golden(golden_dir, tag, tol):
+def test_train_model_multi_feature_golden(golden, tag, tol):
     # the f32 goldens were fitted by sklearn in float32; the oracle is float64 -> looser bound
-    g = _load(golden_dir, f"sk_train_model_{tag}.npz")
+    g = golden(f"sk_train_model_{tag}.npz")
     out = orc.train_model(g["X"], g["y"])
     assert np.max(np.abs(out["coef"] - g["coef"])) < tol
     assert out["rank"] == int(g["rank"])
