@@ -52,6 +52,7 @@ _SIGNATURES = {
     "b2_gram_allreduce": (C.c_int, [_vp]),
     "b2_gram_export": (C.c_int, [_vp, _vp, C.POINTER(_c_i64)]),
     "b2_gram_import": (C.c_int, [_vp, _vp, C.c_int]),
+    "b2_gram_kernels": (C.c_int, [_vp, C.POINTER(C.c_int)]),
     "b2_split_mask": (C.c_int, [_c_i64, _c_i64, C.c_uint32, _vp]),
     "b2_copy_d2d": (C.c_int, [_vp, _vp, _vp, C.c_size_t]),
     "b2_pack_columns": (C.c_int, [_vp, _vp, C.c_int, _c_i64, C.c_int, _vp]),
@@ -257,6 +258,8 @@ class Context:
         self._h = h.value
         self.device = int(device)
         self.d = 0
+        self.kernel = KERNEL_AUTO
+        self.precision = PRECISION_SPLIT
         self.serial = 0      # bumped whenever the resident statistic S changes owner / content (estimators check it)
 
     # -- lifecycle -----------------------------------------------------------------------------
@@ -282,10 +285,12 @@ class Context:
 
     def set_kernel(self, kernel: int) -> None:
         _check(load().b2_ctx_set_kernel(self._h, int(kernel)), "b2_ctx_set_kernel")
+        self.kernel = int(kernel)
 
     def set_precision(self, precision: int) -> None:
         """PRECISION_SPLIT (default, bf16 hi+lo operands) or PRECISION_BF16 (single bf16 operand, 'bf16-accum')."""
         _check(load().b2_ctx_set_precision(self._h, int(precision)), "b2_ctx_set_precision")
+        self.precision = int(precision)
 
     def set_sm_limit(self, n_sms: int) -> None:
         _check(load().b2_ctx_set_sm_limit(self._h, int(n_sms)), "b2_ctx_set_sm_limit")
@@ -369,6 +374,13 @@ class Context:
         _check(load().b2_gram_import(self._h, S.ctypes.data, d), "b2_gram_import")
         self.d = d
         self.serial += 1
+
+    def gram_kernels(self) -> int:
+        """OR of ``1 << KERNEL_*`` of the kernels that added to the resident statistic since the last reset / import /
+        fit (b2_gram_kernels)."""
+        k = C.c_int(0)
+        _check(load().b2_gram_kernels(self._h, C.byref(k)), "b2_gram_kernels")
+        return int(k.value)
 
     def fit(self, X, y, row_mask=None, mask_keep: int = 1, alpha: float = 0.0,
             fit_intercept: bool = True) -> Tuple[np.ndarray, float]:

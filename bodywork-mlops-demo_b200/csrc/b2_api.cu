@@ -124,6 +124,7 @@ int gram_block(b2_ctx* ctx, const void* X, int x_dtype, const float* y, int64_t 
     if (nw_ok && n >= 4096) mode = B2_KERNEL_NARROW;
     else mode = (tc_ok && n >= 2048) ? B2_KERNEL_TCGEN05 : B2_KERNEL_SIMT;
   }
+  ctx->s_kernels |= 1 << mode;
   if (mode == B2_KERNEL_NARROW) return launch_gram_narrow(ctx, X, x_dtype, y, n, d, ldx, mask, keep);
   if (mode == B2_KERNEL_TCGEN05) return launch_gram_tc(ctx, X, x_dtype, y, n, d, ldx, mask, keep);
   return launch_gram_simt(ctx, X, x_dtype, y, n, d, ldx, mask, keep);
@@ -285,7 +286,7 @@ static int ctx_allocate(b2_ctx* ctx) {
   B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->tc_part), sizeof(double) * (size_t)ctx->sm_count * kTcAccElems));
   B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->tc_side), sizeof(double) * (size_t)ctx->sm_count * kTcSideDoubles));
   B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->tc_red), sizeof(double) * (kTcAccElems + 16 + kMaxD + 8)));
-  B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->shift), sizeof(float) * 64 * (kMaxD + 1)));
+  B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->shift), sizeof(float) * kShiftFloats));
   B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->simt_part), sizeof(double) * (size_t)ctx->simt_ctas * kMaxS * kMaxS));
   B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->score_part), sizeof(double) * ((size_t)ctx->score_ctas + 2) * 10));
   B2_CUDA(cudaMalloc(reinterpret_cast<void**>(&ctx->coef_dev), sizeof(double) * (kMaxD + 1)));
@@ -297,7 +298,7 @@ static int ctx_allocate(b2_ctx* ctx) {
   ctx->xchg_status_host[0] = 0u;
   B2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&ctx->coef_host), 2 * sizeof(double) * (kMaxD + 1), cudaHostAllocDefault));
   for (int b = 0; b < 2; ++b) B2_CUDA(cudaEventCreateWithFlags(&ctx->ev_coef[b], cudaEventDisableTiming));
-  B2_CUDA(cudaMemset(ctx->shift, 0, sizeof(float) * 64 * (kMaxD + 1)));
+  B2_CUDA(cudaMemset(ctx->shift, 0, sizeof(float) * kShiftFloats));
   B2_CUDA(cudaMemset(ctx->S, 0, sizeof(double) * kMaxS * kMaxS));
   B2_CUDA(cudaMemset(ctx->tc_side, 0, sizeof(double) * (size_t)ctx->sm_count * kTcSideDoubles));
   B2_CUDA(cudaMemset(ctx->tc_red, 0, sizeof(double) * (kTcAccElems + 16 + kMaxD + 8)));
@@ -527,7 +528,14 @@ int b2_gram_reset(b2_ctx* ctx, int d) {
   if (int r = use_device(ctx)) return r;
   if (d < 1 || d > kMaxD) { set_error("d=%d out of range [1,%d]", d, kMaxD); return B2_E_ARG; }
   ctx->d = d;
+  ctx->s_kernels = 0;
   ctx->s_zero_pending = true;   // cleared (or overwritten) by the first kernel that adds to S: one launch less per fit
+  return B2_OK;
+}
+
+int b2_gram_kernels(b2_ctx* ctx, int* kernels_out) {
+  if (ctx == nullptr || kernels_out == nullptr) { set_error("bad arguments to b2_gram_kernels"); return B2_E_ARG; }
+  *kernels_out = ctx->s_kernels;
   return B2_OK;
 }
 
@@ -625,6 +633,7 @@ int b2_gram_import(b2_ctx* ctx, const double* S_in, int d) {
   if (int r = use_device(ctx)) return r;
   if (d < 1 || d > kMaxD || S_in == nullptr) { set_error("bad arguments to b2_gram_import"); return B2_E_ARG; }
   ctx->d = d;
+  ctx->s_kernels = 0;
   ctx->s_zero_pending = false;
   B2_CUDA(cudaMemsetAsync(ctx->S, 0, sizeof(double) * kMaxS * kMaxS, ctx->stream));
   B2_CUDA(cudaMemcpyAsync(ctx->S, S_in, sizeof(double) * (d + 2) * (d + 2), cudaMemcpyHostToDevice, ctx->stream));
@@ -741,8 +750,10 @@ int b2_fit(b2_ctx* ctx, const void* X, int x_dtype, const float* y, int64_t n_ro
   }
   ctx->d = d;
   ctx->k_launches = 0;
+  ctx->s_kernels = 1 << B2_KERNEL_TCGEN05;
   const int es = x_dtype == B2_F32 ? 4 : 2;
   const int64_t n_main = gram_tc_main_rows(n_rows, d, ldx, nullptr);
+  if (n_main < n_rows) ctx->s_kernels |= 1 << B2_KERNEL_SIMT;
   TcFuse fuse;
   fuse.assign = 1; fuse.scatter = 0; fuse.epoch = 0;
   if (n_main < n_rows) {   // the few rows the packed layout leaves over go in first; the fused fold then adds to S

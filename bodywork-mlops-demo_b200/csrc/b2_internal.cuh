@@ -25,6 +25,7 @@ constexpr int kTcN = 144;                // MMA N: 128 feature columns (hi) + 16
 constexpr int kTcAccCols = 2 * kTcN;     // two accumulators: A = hi and A = lo against the same B = [hi | E]
 constexpr int kTcAccElems = kTcM * kTcAccCols;  // fp32 accumulators drained per chunk (36 864)
 constexpr int kTcSideDoubles = 8;        // per-CTA CUDA-core sums: sum y', sum y'^2, rows used
+constexpr int kShiftFloats = 64 * (kMaxD + 2);   // b2_ctx::shift: 64 partials of the shift sample (features, y, rows)
 
 void set_error(const char* fmt, ...);
 
@@ -57,13 +58,14 @@ struct b2_ctx {
   int precision = B2_PRECISION_SPLIT;
 
   int d = 0;                           // feature count of the current statistic (0 = not reset)
+  int s_kernels = 0;                   // 1 << B2_KERNEL_* of every kernel that added to S since the last reset / import
   double* S = nullptr;                 // device, kMaxS*kMaxS (only (d+2)^2 used, row stride d+2)
 
   // tcgen05 path scratch
   double* tc_part = nullptr;           // [sm_count][kTcAccElems]   per-CTA fp64 partial Gram (col-major)
   double* tc_side = nullptr;           // [sm_count][kTcSideDoubles]
   double* tc_red = nullptr;            // [kTcAccElems + 16 + 129 + pad]: reduced partials, y sums, barrier slot, shift
-  float* shift = nullptr;              // [64][kMaxD + 1] partial sums of the row sample -> per-column shift c
+  float* shift = nullptr;              // [kShiftFloats] partial sums of the row sample -> per-column shift c
   bool tc_attr_set = false;
   bool solve_attr_set = false;
   double* solve_host = nullptr;        // pinned mirror of solve_out (D2H without a staging copy)

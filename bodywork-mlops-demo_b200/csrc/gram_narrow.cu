@@ -66,24 +66,31 @@ __device__ __forceinline__ float shfl_bfly_ordered(float v, int off) {
   return r;
 }
 
-// ---- per-column shift: mean of a strided row sample (any c is algebraically exact, see narrow_fold_kernel) --------
+// ---- per-column shift: mean of a strided sample of the kept rows (any c is algebraically exact, see
+// narrow_fold_kernel).  Dropped rows and non-finite values are skipped and the mean divides by what was summed (nothing
+// summed: c = 0): a masked-out row may hold anything, and a NaN there must not become c. ----------------------------
 template <typename T>
-__global__ void narrow_shift_kernel(const T* __restrict__ X, const float* __restrict__ y, int64_t n, int d,
-                                    float* __restrict__ cvec) {
+__global__ void narrow_shift_kernel(const T* __restrict__ X, const float* __restrict__ y, const uint8_t* __restrict__ mask,
+                                    int keep, int64_t n, int d, float* __restrict__ cvec) {
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;   // warp w: feature w (w < d), warp d: y
   if (w > kNwMaxDP) return;
   if (w > d) { if (lane == 0 && w < kNwMaxDP) cvec[w] = 0.f; return; }
   const int64_t samples = n < kNwShiftSamples ? n : kNwShiftSamples;
   const int64_t stride = n / samples;
-  float acc = 0.f;
+  float acc = 0.f, cnt = 0.f;
   for (int64_t s = lane; s < samples; s += 32) {
     const int64_t row = s * stride;
-    acc += (w < d) ? raw_ld_global<T>(X + row * d + w) : __ldg(y + row);
+    if (mask != nullptr && mask[row] != (uint8_t)keep) continue;
+    const float v = (w < d) ? raw_ld_global<T>(X + row * d + w) : __ldg(y + row);
+    if (fabsf(v) <= 3.0e38f) { acc += v; cnt += 1.f; }
   }
 #pragma unroll
-  for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+  for (int off = 16; off > 0; off >>= 1) {
+    acc += __shfl_xor_sync(0xffffffffu, acc, off);
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, off);
+  }
   if (lane == 0) {
-    cvec[w < d ? w : kNwCY] = acc / (float)samples;
+    cvec[w < d ? w : kNwCY] = cnt > 0.f ? acc / cnt : 0.f;
     if (w == d && d < kNwMaxDP) cvec[d] = 0.f;
   }
 }
@@ -468,7 +475,7 @@ int launch_narrow_t(b2_ctx* ctx, const T* X, const float* y, const uint8_t* mask
   const int n_tiles = (int)(n / rows);            // n <= INT32_MAX rows (gram_narrow_supported)
   *rows_done = (int64_t)n_tiles * rows;
   if (n_tiles == 0) return B2_OK;
-  narrow_shift_kernel<T><<<1, 32 * (kNwMaxDP + 1), 0, ctx->stream>>>(X, y, n, d, ctx->shift);
+  narrow_shift_kernel<T><<<1, 32 * (kNwMaxDP + 1), 0, ctx->stream>>>(X, y, mask, keep, n, d, ctx->shift);
   B2_CUDA(cudaGetLastError());
   const int pair = ctx->k_pairs % kKernelEventPairs;
   B2_CUDA(cudaEventRecord(ctx->ev_k[pair][0], ctx->stream));

@@ -163,32 +163,46 @@ __device__ __forceinline__ void split2(float v0, float v1, uint32_t& hi, uint32_
 }
 
 // ------------------------------------------------------------------------------------------
-// per-column shift c: mean of a strided row sample (any value near the column mean will do;
-// the algebra in tc_fold_kernel is exact for every c)
+// per-column shift c: mean of a strided sample of the rows the statistic keeps (any value near the column mean will
+// do; the algebra in tc_fold_kernel is exact for every c)
 // ------------------------------------------------------------------------------------------
 constexpr int kShiftBlocks = 64;                 // partial sums of the row sample, one per block
-constexpr int kShiftStride = kMaxD + 1;          // floats per partial: features, then y (slot kMaxD)
+constexpr int kShiftStride = kMaxD + 2;          // floats per partial: features, y (slot kMaxD), rows sampled (kMaxD + 1)
+static_assert(kShiftBlocks * kShiftStride <= kShiftFloats, "b2_ctx::shift holds the partials");
 
 __host__ __device__ __forceinline__ int64_t shift_samples(int64_t n) { return n < 2048 ? n : 2048; }
 
-// c_j from the 64 partial sums; bf16-representable so that (bf16 input - c) is exact in fp32.
-// Called with identical arguments by the Gram kernel and by tc_fold_kernel -> identical c.
-__device__ __forceinline__ float shift_value(const float* __restrict__ sp, int j, int64_t n) {
-  float acc = 0.f;
+// c_j from the column's sum over the sampled rows and their count (no row sampled: c = 0).  fp32 rows take the fp32
+// mean: x - c is exact when the offset dominates (Sterbenz) and rounds at 2^-24 |x - c| otherwise, far below the hi/lo
+// split's 2^-17 -- whereas a bf16-rounded c leaves a residual mean - c of up to half a bf16 spacing (32 for a column
+// at 10016), and every shifted value carries it into the fp32 sums.  The bf16-storage kernels need c on the bf16 grid
+// (they subtract it in bf16; the single-operand kernel feeds the raw tile to the tensor core): `bf16_grid`.
+__device__ __forceinline__ float shift_from_sums(float sum, float rows, bool bf16_grid) {
+  const float c = rows > 0.f ? sum / rows : 0.f;
+  return bf16_grid ? __bfloat162float(__float2bfloat16_rn(c)) : c;
+}
+// Called with identical arguments by the Gram kernels and (on its shared-memory copy of the partials, same order of
+// the 64 additions) by tc_finalize_kernel -> identical c.
+__device__ __forceinline__ float shift_value(const float* __restrict__ sp, int j, bool bf16_grid) {
+  float acc = 0.f, rows = 0.f;
 #pragma unroll 8
-  for (int b = 0; b < kShiftBlocks; ++b) acc += sp[b * kShiftStride + j];
-  return __bfloat162float(__float2bfloat16_rn(acc / (float)shift_samples(n)));
+  for (int b = 0; b < kShiftBlocks; ++b) {
+    acc += sp[b * kShiftStride + j];
+    rows += sp[b * kShiftStride + kMaxD + 1];
+  }
+  return shift_from_sums(acc, rows, bf16_grid);
 }
 
 // 64 blocks x (4 row groups x 160 columns): a thread sums 8 sample rows (one batch of loads in flight -- the rows are
-// megabytes apart, every load is a DRAM round trip), the 4 groups are combined in a fixed order.
-constexpr int kShiftCols = 160;                  // >= kMaxD + 1, a multiple of 32
+// megabytes apart, every load is a DRAM round trip), the 4 groups are combined in a fixed order.  Column d + 1 counts
+// the sampled rows the mask keeps; a dropped row contributes nothing, whatever it holds.
+constexpr int kShiftCols = 160;                  // >= kMaxD + 2, a multiple of 32
 constexpr int kShiftGroups = 4;
 
 template <typename T>
 __global__ void __launch_bounds__(kShiftCols * kShiftGroups)
-tc_shift_kernel(const T* __restrict__ X, const float* __restrict__ y, int64_t n, int d,
-                int64_t ldx, float* __restrict__ sp) {
+tc_shift_kernel(const T* __restrict__ X, const float* __restrict__ y, const uint8_t* __restrict__ mask, int keep,
+                int64_t n, int d, int64_t ldx, float* __restrict__ sp) {
   __shared__ float sub[kShiftGroups][kShiftCols];
   const int j = threadIdx.x % kShiftCols, g = threadIdx.x / kShiftCols;
   const int64_t samples = shift_samples(n);
@@ -197,17 +211,19 @@ tc_shift_kernel(const T* __restrict__ X, const float* __restrict__ y, int64_t n,
   const int64_t s0 = blockIdx.x * per;
   const int64_t s1 = (s0 + per < samples) ? s0 + per : samples;
   float acc = 0.f;
-  if (j <= d) {
+  if (j <= d + 1) {
 #pragma unroll 8
     for (int64_t s = s0 + g; s < s1; s += kShiftGroups) {
       const int64_t row = s * stride;
-      const float v = (j < d) ? raw_ld_global<T>(X + row * ldx + j) : __ldg(y + row);
-      acc += (fabsf(v) <= 3.0e38f) ? v : 0.f;     // the sample ignores the row mask: a dropped row may hold NaN / Inf
+      if (mask != nullptr && mask[row] != (uint8_t)keep) continue;
+      const float v = (j < d) ? raw_ld_global<T>(X + row * ldx + j) : (j == d ? __ldg(y + row) : 1.f);
+      acc += (fabsf(v) <= 3.0e38f) ? v : 0.f;     // a kept non-finite value makes the statistic non-finite anyway
     }
   }
   sub[g][j] = acc;
   __syncthreads();
-  if (g == 0 && j <= d) sp[blockIdx.x * kShiftStride + (j == d ? kMaxD : j)] = ((sub[0][j] + sub[1][j]) + sub[2][j]) + sub[3][j];
+  if (g == 0 && j <= d + 1)
+    sp[blockIdx.x * kShiftStride + (j < d ? j : kMaxD + (j - d))] = ((sub[0][j] + sub[1][j]) + sub[2][j]) + sub[3][j];
 }
 
 // ------------------------------------------------------------------------------------------
@@ -288,7 +304,8 @@ __device__ __forceinline__ void grid_barrier(unsigned int* ctr) {
 template <typename CT>
 __device__ __forceinline__ double tc_fold_value(const double* red, const CT* c, int d, int pack, int idx) {
   const int dp = d + 2;
-  const int a = idx / dp, b = idx % dp;
+  const int r = idx / dp, q = idx % dp;
+  const int a = r < q ? r : q, b = r < q ? q : r;   // (a, b) and (b, a) evaluate the same expression: S stays bit-symmetric
   // D1[i][j] = red[j*128 + i], D2[i][j] = red[(144 + j)*128 + i]
   auto D1 = [&](int i, int j) { return __ldcg(red + (size_t)j * kTcM + i); };
   auto D2 = [&](int i, int j) { return __ldcg(red + (size_t)(kTcN + j) * kTcM + i); };
@@ -348,7 +365,7 @@ template <typename T, int DFIX, bool SPLIT>
 __global__ void __launch_bounds__(kThreads, 1)
 gram_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmY,
                const __grid_constant__ CUtensorMap tmM, int y_map_2d, int has_mask, int keep,
-               int64_t n_rows, int d_arg, int pack, int d_orig, int64_t n_shift, const float* __restrict__ shift,
+               int64_t n_rows, int d_arg, int pack, int d_orig, const float* __restrict__ shift,
                int chunk_tiles,
                double* __restrict__ part, double* __restrict__ side, uint32_t wait_ns, uint32_t dbg_arg) {
 #ifdef B2_DEV_KNOBS
@@ -414,8 +431,8 @@ gram_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
   // packed rows (pack > 1): super-row feature i < pack * d_orig is original feature i % d_orig -> the shift repeats;
   // the columns from pack * d_orig to 127 are TMA out-of-bounds zero fill and keep shift 0 (they contribute nothing)
   for (int j = threadIdx.x; j <= kMaxD; j += kThreads)
-    shift_s[j] = (j == kMaxD) ? shift_value(shift, kMaxD, n_shift)
-                              : (j < pack * d_orig ? shift_value(shift, j % d_orig, n_shift) : 0.f);
+    shift_s[j] = (j == kMaxD) ? shift_value(shift, kMaxD, false)
+                              : (j < pack * d_orig ? shift_value(shift, j % d_orig, false) : 0.f);
   fence_proxy_async_smem();
   tc_fence_before();
   __syncthreads();
@@ -713,7 +730,7 @@ constexpr int kFinalizeCtas = (kRedElems + kFinalizeThreads / 4 - 1) / (kFinaliz
 
 __global__ void __launch_bounds__(kFinalizeThreads, 1)
 tc_finalize_kernel(const double* part, const double* side, int n_ctas, double* red, const float* __restrict__ shift,
-                   int64_t n_rows, int d, int pack, double* S, unsigned int* sync, const TcFinal fin) {
+                   int bf16_grid, int d, int pack, double* S, unsigned int* sync, const TcFinal fin) {
   __shared__ double quarter[kFinalizeThreads];
   __shared__ double c_s[kMaxD + 1];                              // the shift as fp64 (c_s[kMaxD]: c_y)
   __shared__ float c_part[kShiftBlocks * kShiftStride];          // the 64 partial sums of the shift sample (33 KB)
@@ -723,10 +740,13 @@ tc_finalize_kernel(const double* part, const double* side, int n_ctas, double* r
   for (int idx = threadIdx.x; idx < kShiftBlocks * kShiftStride; idx += blockDim.x) c_part[idx] = __ldg(shift + idx);
   __syncthreads();
   for (int j = threadIdx.x; j <= kMaxD; j += blockDim.x) {
-    float acc = 0.f;
+    float acc = 0.f, rows = 0.f;
 #pragma unroll 8
-    for (int b = 0; b < kShiftBlocks; ++b) acc += c_part[b * kShiftStride + j];
-    c_s[j] = (j < d || j == kMaxD) ? (double)__bfloat162float(__float2bfloat16_rn(acc / (float)shift_samples(n_rows))) : 0.0;
+    for (int b = 0; b < kShiftBlocks; ++b) {
+      acc += c_part[b * kShiftStride + j];
+      rows += c_part[b * kShiftStride + kMaxD + 1];
+    }
+    c_s[j] = (j < d || j == kMaxD) ? (double)shift_from_sums(acc, rows, bf16_grid != 0 && j < kMaxD) : 0.0;
   }
   {
     constexpr int epb = kFinalizeThreads / 4;                    // elements per pass of a CTA
@@ -957,11 +977,11 @@ int launch_gram_tc(b2_ctx* ctx, const void* X, int x_dtype, const float* y, int6
     if (int r = ensure_s_cleared(ctx)) return r;
   }
   if (x_dtype == B2_F32)
-    tc_shift_kernel<float><<<kShiftBlocks, kShiftCols * kShiftGroups, 0, ctx->stream>>>(static_cast<const float*>(X), y, n_in, d_in,
-                                                                  ldx_in, ctx->shift);
+    tc_shift_kernel<float><<<kShiftBlocks, kShiftCols * kShiftGroups, 0, ctx->stream>>>(static_cast<const float*>(X), y, mask, keep,
+                                                                                          n_in, d_in, ldx_in, ctx->shift);
   else
-    tc_shift_kernel<__nv_bfloat16><<<kShiftBlocks, kShiftCols * kShiftGroups, 0, ctx->stream>>>(static_cast<const __nv_bfloat16*>(X), y,
-                                                                          n_in, d_in, ldx_in, ctx->shift);
+    tc_shift_kernel<__nv_bfloat16><<<kShiftBlocks, kShiftCols * kShiftGroups, 0, ctx->stream>>>(
+        static_cast<const __nv_bfloat16*>(X), y, mask, keep, n_in, d_in, ldx_in, ctx->shift);
   B2_CUDA(cudaGetLastError());
 
 #ifdef B2_DEV_KNOBS
@@ -984,7 +1004,7 @@ int launch_gram_tc(b2_ctx* ctx, const void* X, int x_dtype, const float* y, int6
   B2_CUDA(cudaEventRecord(ctx->ev_k[pair][0], ctx->stream));
 #define B2_LAUNCH_TC(T, DF, SP)                                                                          \
   gram_tc_kernel<T, DF, SP><<<grid, kThreads, kSmemBytes, ctx->stream>>>(                                \
-      tmX, tmY, tmM, y_map_2d, mask != nullptr ? 1 + m_map_2d : 0, keep, n, d, pack, d_in, n_in, ctx->shift, \
+      tmX, tmY, tmM, y_map_2d, mask != nullptr ? 1 + m_map_2d : 0, keep, n, d, pack, d_in, ctx->shift,       \
       chunk_tiles,                                                                                        \
       ctx->tc_part, ctx->tc_side, wait_ns, dbg)
 #define B2_LAUNCH_TC_D(T, SP) \
@@ -993,10 +1013,10 @@ int launch_gram_tc(b2_ctx* ctx, const void* X, int x_dtype, const float* y, int6
   if (b16) {
     const int hm = mask != nullptr ? 1 + m_map_2d : 0;
     if (split)
-      b16::sp::gram_b16_split_kernel<<<grid, kThreads, b16::sp::kSmem, ctx->stream>>>(tmX, tmY, tmM, y_map_2d, hm, keep, n, n_in,
+      b16::sp::gram_b16_split_kernel<<<grid, kThreads, b16::sp::kSmem, ctx->stream>>>(tmX, tmY, tmM, y_map_2d, hm, keep, n,
                                                                                       ctx->shift, chunk_tiles, ctx->tc_part, ctx->tc_side);
     else
-      b16::gram_b16_single_kernel<<<grid, kThreads, b16::kSmem, ctx->stream>>>(tmX, tmY, tmM, y_map_2d, hm, keep, n, n_in, ctx->shift,
+      b16::gram_b16_single_kernel<<<grid, kThreads, b16::kSmem, ctx->stream>>>(tmX, tmY, tmM, y_map_2d, hm, keep, n, ctx->shift,
                                                                                chunk_tiles, ctx->tc_part, ctx->tc_side);
   } else if (x_dtype == B2_F32) {
     if (split) B2_LAUNCH_TC_D(float, true); else B2_LAUNCH_TC_D(float, false);
@@ -1029,8 +1049,8 @@ int launch_gram_tc(b2_ctx* ctx, const void* X, int x_dtype, const float* y, int6
     cfg.attrs = attr; cfg.numAttrs = 1;
     const double* part_arg = ctx->tc_part; const double* side_arg = ctx->tc_side;
     const float* shift_arg = ctx->shift;
-    B2_CUDA(cudaLaunchKernelEx(&cfg, tc_finalize_kernel, part_arg, side_arg, grid, ctx->tc_red, shift_arg, n_in, d_in, pack,
-                               ctx->S, ctx->tc_sync, fin));
+    B2_CUDA(cudaLaunchKernelEx(&cfg, tc_finalize_kernel, part_arg, side_arg, grid, ctx->tc_red, shift_arg, b16 ? 1 : 0, d_in,
+                               pack, ctx->S, ctx->tc_sync, fin));
   }
   ctx->launches += 3;
   ctx->k_launches += 3;

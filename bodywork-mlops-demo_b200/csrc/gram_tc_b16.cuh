@@ -175,7 +175,7 @@ __device__ __forceinline__ bool issue_tile_single(uint32_t tmem_acc, uint32_t tm
 __global__ void __launch_bounds__(kThreads, 1)
 gram_b16_single_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmY,
                 const __grid_constant__ CUtensorMap tmM, int y_map_2d, int has_mask, int keep, int64_t n_rows,
-                int64_t n_shift, const float* __restrict__ shift, int chunk_tiles, double* __restrict__ part,
+                const float* __restrict__ shift, int chunk_tiles, double* __restrict__ part,
                 double* __restrict__ side) {
   constexpr int kOps = kOpsMax;
   extern __shared__ uint8_t smem_raw[];
@@ -227,7 +227,7 @@ gram_b16_single_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_con
   for (int st = 0; st < kRaw; ++st)
     for (uint32_t o = threadIdx.x * 16; o < kRawHalf; o += kThreads * 16)
       *reinterpret_cast<uint4*>(smem + kOffRaw + st * kRawBytes + kRawX + o) = make_uint4(0, 0, 0, 0);
-  for (int j = threadIdx.x; j <= kMaxD; j += kThreads) shift_s[j] = shift_value(shift, j, n_shift);
+  for (int j = threadIdx.x; j <= kMaxD; j += kThreads) shift_s[j] = shift_value(shift, j, j < kMaxD);   // c_y: fp32
   fence_proxy_async_smem();
   tc_fence_before();
   __syncthreads();

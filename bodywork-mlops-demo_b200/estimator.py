@@ -30,6 +30,14 @@ def default_context() -> native.Context:
 
 _F64_UPLOAD_LIMIT = 64 << 30     # float64 host rows larger than this (as fp32, bytes) are converted and streamed block-wise
 
+# Smallest sqrt(lambda_min / lambda_max) of the centred Gram, scaled to unit diagonal, that a statistic from an inexact
+# kernel resolves.  The kernels' error is entrywise relative, |dA_ij| <= eps sqrt(A_ii A_jj) (tests/test_gpu_hard_data.py:
+# tensor core ~3e-5, narrow ~3e-7), i.e. eps in the scaled matrix, whatever the column scales; the limits are ~sqrt of
+# eps * D.  Below them the small eigenvalues are noise of either sign, so neither the LDL^T pivots nor rank_ can be
+# trusted.
+_RESOLVABLE = {native.KERNEL_NARROW: 3e-3, native.KERNEL_TCGEN05: 1e-2}
+_RESOLVABLE_BF16_OPERAND = 1e-1      # the tensor core's single-operand mode (PRECISION_BF16)
+
 
 def _as_f32_matrix(X) -> np.ndarray:
     X = np.asarray(X)
@@ -89,10 +97,76 @@ class B200LinearRegression:
             if hasattr(self, name):
                 delattr(self, name)
 
+    def _unresolved(self) -> bool:
+        """Did an inexact kernel build the resident statistic, and is its centred Gram closer to singular than that
+        kernel resolves?  Judged on the Gram scaled to unit diagonal (the kernels' error is relative to the columns' own
+        scales), so a well-conditioned design whose columns differ in scale -- age beside income -- keeps the fast
+        statistic.  With a communicator the decision must be the same on every rank (the rebuild all-reduces): it then
+        depends on the all-reduced S alone and takes the largest limit, whichever kernels this rank's shard used."""
+        ctx = self.ctx
+        if ctx.comm_info()["n_ranks"] > 1:
+            limit = max(max(_RESOLVABLE.values()), _RESOLVABLE_BF16_OPERAND)
+        else:
+            used = ctx.gram_kernels()
+            limits = [lim for k, lim in _RESOLVABLE.items() if used & (1 << k)]
+            if used & (1 << native.KERNEL_TCGEN05) and ctx.precision == native.PRECISION_BF16:
+                limits.append(_RESOLVABLE_BF16_OPERAND)
+            if not limits:
+                return False
+            limit = max(limits)
+        s = np.asarray(getattr(self, "singular_", ()))
+        if s.size < 2 or not s[0] > 0.0 or s[-1] >= limit * np.sqrt(s.size) * s[0]:
+            return False       # van der Sluis: kappa(scaled) <= D kappa(unscaled), so the scaled Gram is resolved too
+        # the unscaled spectrum is near singular: look at the scaled one (host eigvalsh of a D x D matrix, ~1 ms at 128)
+        S = ctx.gram_export()
+        d = S.shape[0] - 2
+        n = S[d, d]
+        if self.fit_intercept:
+            xm = S[:d, d] / n
+            A = S[:d, :d] - n * np.outer(xm, xm)
+        else:
+            A = S[:d, :d].copy()
+        dg = np.diag(A).copy()
+        # a column whose centred variance is at the fp64 rounding of its raw moment is constant: no scale to judge by
+        if np.any(dg <= 64.0 * np.finfo(np.float64).eps * np.abs(np.diag(S)[:d])):
+            return True
+        r = 1.0 / np.sqrt(dg)
+        lam = np.linalg.eigvalsh(0.5 * (A + A.T) * np.outer(r, r))
+        return not lam[0] > (limit ** 2) * lam[-1]
+
+    def _refit_exact(self, X, y, row_mask, mask_keep, d: int) -> None:
+        """Rebuild the statistic of the same rows on the exact fp64 kernel and solve again."""
+        ctx = self.ctx
+        kernel = ctx.kernel
+        ctx.set_kernel(native.KERNEL_SIMT)
+        try:
+            ctx.gram_reset(d)
+            ctx.gram_accumulate(X, y, row_mask, mask_keep)
+            ctx.gram_allreduce()
+        finally:
+            ctx.set_kernel(kernel)
+        self._drop_spectrum()
+        singular = False
+        try:
+            coef, b0 = ctx.solve(alpha=self.alpha, fit_intercept=self.fit_intercept)
+            self._set_solution(coef, b0, d)
+        except np.linalg.LinAlgError:
+            singular = True
+        self._serial = ctx.serial
+        self._spectrum(d, need_coef=singular)
+
     def fit(self, X, y, row_mask=None, mask_keep: int = 1, with_spectrum: bool = True) -> "B200LinearRegression":
         """X: (n, D) host array (any float dtype; staged as fp32) or a ``DeviceArray`` (f32 / bf16).
         ``row_mask`` (uint8 per row) restricts the fit to rows equal to ``mask_keep``.
-        ``with_spectrum=False`` defers ``singular_`` / ``rank_`` (computed on first use, e.g. by ``to_sklearn``)."""
+        ``with_spectrum=False`` defers ``singular_`` / ``rank_`` (computed on first use, e.g. by ``to_sklearn``).
+
+        When the tensor-core or narrow kernel built the statistic and its spectrum shows the centred Gram closer to
+        singular than that kernel resolves (s_min / s_max below ~sqrt of its error), the rows are accumulated again on
+        the exact fp64 kernel and solved from that statistic: rank_, coef_ and singular_ are then gelsd's even for an
+        exactly collinear design (one-hot blocks with the intercept, x2 = 3 x1, ...).  "Near singular" is judged on the
+        Gram scaled to unit diagonal: well-conditioned fits never pay for it, however different their columns' scales.  The check needs the spectrum: with ``with_spectrum=False`` the fit keeps the inexact statistic's
+        solution (and the deferred spectrum is that statistic's); ``partial_fit`` and ``solve_resident`` no longer hold
+        the earlier tranches' rows and likewise solve what the kernels accumulated."""
         ctx = self.ctx
         owned = []                  # device buffers this call created (float64 host rows: converted on the way up)
         if isinstance(X, native.DeviceArray):
@@ -121,18 +195,21 @@ class B200LinearRegression:
             d = X.shape[1]
         self._S = None
         self._drop_spectrum()
-        singular = False
         try:
-            coef, b0 = ctx.fit(X, y, row_mask, mask_keep, alpha=self.alpha, fit_intercept=self.fit_intercept)
-            self._set_solution(coef, b0, d)
-        except np.linalg.LinAlgError:
-            singular = True         # rank deficient and alpha == 0: the minimum-norm solution gelsd would return
+            singular = False
+            try:
+                coef, b0 = ctx.fit(X, y, row_mask, mask_keep, alpha=self.alpha, fit_intercept=self.fit_intercept)
+                self._set_solution(coef, b0, d)
+            except np.linalg.LinAlgError:
+                singular = True     # rank deficient and alpha == 0: the minimum-norm solution gelsd would return
+            self._serial = ctx.serial
+            if with_spectrum or singular:
+                self._spectrum(d, need_coef=singular)
+                if self._unresolved():
+                    self._refit_exact(X, y, row_mask, mask_keep, d)
         finally:
             for a in owned:
                 a.free()
-        self._serial = ctx.serial
-        if with_spectrum or singular:
-            self._spectrum(d, need_coef=singular)
         return self
 
     def partial_fit(self, X, y, with_spectrum: bool = False) -> "B200LinearRegression":

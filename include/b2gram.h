@@ -125,6 +125,11 @@ int b2_gram_allreduce(b2_ctx* ctx);
 /* copy S out / in (incremental-refit state).  S_out/S_in: (d+2)^2 doubles on the host */
 int b2_gram_export(b2_ctx* ctx, double* S_out, int64_t* n_rows_out);
 int b2_gram_import(b2_ctx* ctx, const double* S_in, int d);
+/* which kernel families added to the resident S since the last b2_gram_reset / b2_gram_import / b2_fit:
+ * *kernels_out = OR of (1 << B2_KERNEL_SIMT / _TCGEN05 / _NARROW) (0 after an import: the source is the caller's).
+ * A statistic from the tensor-core or narrow kernel resolves eigenvalues only down to ~eps_kernel of the largest, so a
+ * caller that finds the centred Gram near singular can rebuild S on the exact kernel (B200LinearRegression.fit does). */
+int b2_gram_kernels(b2_ctx* ctx, int* kernels_out);
 
 /* ---- split: the row membership of train_test_split(X, y, test_size, random_state=seed) ---------------------------
  * reference: stage_1_train_model.py:98-103 -> sklearn ShuffleSplit: perm = RandomState(seed).permutation(n_rows);
